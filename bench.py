@@ -237,6 +237,16 @@ def dense_sumcheck_leg(sb, api, sd, ctx, rank, world, pk, logn=22, rounds=5):
             "note": "time = kernel + the device->host copy of the three evaluations (and, sharded, the NVLink exchange of 96 B per rank inside the kernel); frac_of_hbm against N x the measured copy bandwidth"}
 
 
+def dump_outputs(out_dir, proofs):
+    """The proofs the last timed step of each timed region returned, one float32 value per byte (0..255, exact), as <out_dir>/<name>.npy.
+    The instance, assignment, generators, transcript label and random tape are all seeded, so two builds run with the same arguments
+    can be compared output for output.  Rank 0's proofs only; at 2^20 each array holds 180,840 values (~720 KB)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, b in proofs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.frombuffer(b, dtype=np.uint8).astype(np.float32))
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -292,6 +302,7 @@ def run_b200(args):
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     launches = sb.kernel_launches() - launches0
+    proof_resident = proof
     t_res = sum(per_step) / 1e3
     # ---- timed region 2: end to end through the public API with host buffers
     step_e2e()
@@ -308,6 +319,8 @@ def run_b200(args):
     h1, d1 = api.io_bytes()
     t_e2e = sum(per_step_e2e) / 1e3
     t_res, t_e2e = sd.max_over_ranks([t_res, t_e2e])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"proof_bytes": proof_resident.bytes, "proof_bytes_e2e": proof.bytes})
     # ---- roofline leg: CUDA-event timing of every kernel family over one more step (separate from the timed regions above)
     roof = None
     if rank == 0:
@@ -451,7 +464,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-msm-var", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the proof bytes of the last timed step of each timed region to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
